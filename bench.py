@@ -24,6 +24,11 @@ an eager (un-captured) pass over the same step; `roofline_scatter` = the scatter
 shape and inside a C4 step; `cpu_baseline` = the reference's CPU path on this host.  `--impl reference` times that CPU
 path as its own arm (the unmodified reference modules when `baseline/_ref/graphinvent/gnn` is present, else the
 oracle port).
+
+`--dump-outputs DIR` writes what the last of the K timed steps computed (rank 0): `loss`, `logits` [B, APD],
+`grads` (the flat gradient bucket) and `params` (the parameters after that step's Adam update, flattened in
+`named_parameters()` order), as DIR/<name>.npy in float32.  Inputs and initial weights are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -41,6 +46,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the tree may be read-only: no __pycache__ next to the sources
 
 CONFIGS = {
     # name: (constants overrides, batch, atoms, atom types, charges, description)
@@ -55,6 +61,7 @@ CONFIGS = {
     "C5T": (dict(model="EMN"), 1000, 13, 5, 3, "EMN defaults gdb13 dims, batch=1000 (training step of the C5 model)"),
 }
 UNIT = "graphs/s"
+DUMP_LIMIT_BYTES = 64 << 20
 CPU_MICRO_BATCH = 256     # the reference's O(V*E) prologue cannot run the large configurations whole (SURVEY.md 8d)
 REF_DIR = os.path.join(ROOT, "baseline", "_ref", "graphinvent")
 
@@ -322,6 +329,21 @@ def scatter_roofline(pk):
             "l2": "working set 204 MB > 126 MB L2, no flush needed"}
 
 
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """arrays (name -> device tensor) as out_dir/<name>.npy in float32; if they hold more than `limit` bytes together,
+    every array larger than its even share of the limit is replaced by a fixed seeded sample of its flattened elements
+    (sorted indices, the same on every run)"""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    share = limit // len(host)
+    for i, (name, a) in enumerate(host.items()):
+        if total > limit and a.nbytes > share:
+            rng = np.random.default_rng(i)
+            a = a.reshape(-1)[np.sort(rng.choice(a.size, share // 4, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def _flat_grads(net):
     return torch.cat([p.grad.detach().reshape(-1) for p in net.parameters()])
 
@@ -436,19 +458,26 @@ def run_b200_arm(args):
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     final_loss = float(loss)
     step.check()                              # capacity respected (one 64-byte read, outside the timed region)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": step.loss, "logits": step.out, "grads": step.gflat,
+                                         "params": torch.cat([p.detach().reshape(-1) for p in step.params])})
 
-    # ---- timed region 1b: the same step for >= 1 s (a 20-step region is shorter than nvidia-smi's sampling period
-    #      and than the power-cap time constant the sustained tensor peak is quoted under) ----------------------
-    long_steps = max(args.steps, int(math.ceil(args.min_seconds * 1e3 / (ms_total / args.steps))))
-    lv0, lv1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
-    lv0.record()
-    for _ in range(long_steps):
-        loss = step()
-    lv1.record()
-    barrier()
+    # ---- timed region 1b, only with --min-seconds: the same step for that long (a 20-step region is shorter than
+    #      nvidia-smi's sampling period and than the power-cap time constant the sustained tensor peak is quoted under)
+    long_run = None
+    if args.min_seconds > 0:
+        long_steps = max(args.steps, int(math.ceil(args.min_seconds * 1e3 / (ms_total / args.steps))))
+        lv0, lv1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        barrier()
+        lv0.record()
+        for _ in range(long_steps):
+            loss = step()
+        lv1.record()
+        barrier()
+        ms_long = max_over_ranks(lv0.elapsed_time(lv1))
+        long_run = {"steps": long_steps, "ms_per_step": ms_long / long_steps,
+                    "value": global_batch * long_steps / (ms_long / 1e3), "seconds": ms_long / 1e3}
     t_region1 = time.monotonic()
-    ms_long = max_over_ranks(lv0.elapsed_time(lv1))
     clocks = sampler.stop(t_region0, t_region1) if rank == 0 else None
 
     # ---- timed region 2: end to end from pinned host buffers ---------------------------------------------
@@ -631,8 +660,7 @@ def run_b200_arm(args):
                        "l2": "per-step working set (saved activations + packed weights, "
                              f"{step.workspace_bytes / 1e6:.0f} MB) exceeds the 126 MB L2; no explicit flush"
                              if "step" in dir() else "working set exceeds L2"},
-            "long_run": {"steps": long_steps, "ms_per_step": ms_long / long_steps,
-                         "value": global_batch * long_steps / (ms_long / 1e3), "seconds": ms_long / 1e3},
+            "long_run": long_run,
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4,
                     "ms_per_step": ms_e2e / args.steps,
                     "how": "TrainStep(nodes, edges, target) with pinned host tensors: H2D into the static input buffers -> "
@@ -733,13 +761,18 @@ def main():
                          "weak = every rank its own full batch")
     ap.add_argument("--input", default="int8", choices=["int8", "float32"],
                     help="element type of the nodes / edges batches (int8 = the reference's on-disk type)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="length of the additional long timed region")
+    ap.add_argument("--min-seconds", type=float, default=0.0,
+                    help="if > 0, an additional timed region of at least this many seconds (`long_run`)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-module-api", action="store_true")
     ap.add_argument("--no-single", action="store_true", help="N > 1: skip the single-GPU run of the same workload")
     ap.add_argument("--no-k2-in-model", action="store_true")
     ap.add_argument("--launch-table", default=None, help="write the per-launch timing table of the eager pass here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     if args.config is None:
         args.config = "C2" if max(world, args.gpus) == 1 else "C4"

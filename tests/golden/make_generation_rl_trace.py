@@ -1,13 +1,17 @@
 """
 Records a golden trace of the reference's RL rollout generator (`GraphGeneratorRL.build_graphs`, reference
 GraphGeneratorRL.py:109-172) and of the gradient that `Workflow.learning_step` (Workflow.py:569-612) sends back
-through the whole rollout.  Run in the build container:
+through the whole rollout:
 
-    python tests/golden/make_generation_rl_trace.py
+    GRAPHINVENT_REFERENCE=<GraphINVENT checkout> python tests/golden/make_generation_rl_trace.py
 
 The unmodified reference `GraphGeneratorRL` is imported with the stub modules of `make_generation_trace.py`.
-agent = reference GGNN with the shipped checkpoint (train mode, as in learning_step); prior = the same weights
-plus a seeded perturbation (so that the two likelihood streams differ).  Recorded per round: the sampled flat APD
+agent = reference GGNN with tests/conftest.py::pretrained_like_state_dict() (train mode, as in learning_step);
+prior = the same weights plus a seeded perturbation (so that the two likelihood streams differ).  Weights of that kind
+terminate almost every molecule within two rounds, so the draws are not sampled from the agent: the generator is fed
+the draws of generation_rl_trace.npz, which were sampled by the shipped trained checkpoint
+(data/fine-tuning/gdb13_1K-debug/pretrained_model.pth, 16 rounds); the rollout reproduces that trace's buffers, and
+generation_rl_trace_pretrained_like.npz receives what depends on the weights.  Recorded per round: the flat APD
 index and the agent / prior likelihoods the generator stores for it; at the end: the generator's buffers, the
 log-likelihoods `sample()` returns (:92-97, restated without the RDKit conversion), the loss of
 `Workflow.compute_loss_component` (:889-896) on fixed pseudo-scores and, per parameter tensor of both models, the
@@ -33,7 +37,7 @@ PRIOR_SEED, PRIOR_NOISE = 123, 0.02
 
 
 def perturbed(sd, seed=PRIOR_SEED, noise=PRIOR_NOISE):
-    """the prior's weights: checkpoint + noise * randn, tensor by tensor in state_dict order (CPU generator)"""
+    """the prior's weights: agent's + noise * randn, tensor by tensor in state_dict order (CPU generator)"""
     g = torch.Generator().manual_seed(seed)
     return {k: v + noise * torch.randn(v.shape, generator=g) for k, v in sd.items()}
 
@@ -49,7 +53,9 @@ def main(batch=40, seed=11):
     refimpl.load()
     import GraphGeneratorRL as GG                            # the unmodified reference module
     torch.manual_seed(seed)
-    sd = torch.load(os.path.join(HERE, "_local", "pretrained_model.pth"), map_location="cpu", weights_only=False)
+    forced = np.load(os.path.join(HERE, "generation_rl_trace.npz"))["actions"]
+    from tests.conftest import pretrained_like_state_dict
+    sd = pretrained_like_state_dict()
     agent = refimpl.build(O.make_constants("GGNN"))
     agent.load_state_dict(sd)
     prior = copy.deepcopy(agent)
@@ -60,7 +66,8 @@ def main(batch=40, seed=11):
     orig_sample = torch.distributions.Multinomial.sample
 
     def recording_sample(self, sample_shape=torch.Size()):
-        one_hot = orig_sample(self, sample_shape)
+        one_hot = torch.zeros_like(self.probs)
+        one_hot[torch.arange(one_hot.shape[0]), torch.from_numpy(forced[len(draws)]).long()] = 1
         draws.append(one_hot.argmax(1).to(torch.int32).numpy().copy())
         return one_hot
 
@@ -109,7 +116,10 @@ def main(batch=40, seed=11):
                 out[f"grad_{tag}/{k}"] = p.grad.numpy().copy()
         out[f"grad_norm_{tag}"] = np.array(norms, np.float64)
         out[f"grad_names_{tag}"] = np.array(names)
-    np.savez_compressed(os.path.join(HERE, "generation_rl_trace.npz"), **out)
+    # the draws and buffers are those of generation_rl_trace.npz; store what the weights decide
+    keep = {k: v for k, v in out.items()
+            if "likelihood" in k or k.startswith("grad_") or k in ("loss", "sigma", "prior_seed", "prior_noise")}
+    np.savez_compressed(os.path.join(HERE, "generation_rl_trace_pretrained_like.npz"), **keep)
     nn = gen.generated_n_nodes[:n_generated].float()
     print(f"rounds {len(draws)}, generated {n_generated}, properly terminated "
           f"{int(gen.properly_terminated[:n_generated].sum())}, mean atoms {nn.mean():.2f}, max {int(nn.max())}, "

@@ -1,8 +1,8 @@
 """
 Records a golden trace of the reference's batched graph generator (`GraphGenerator.build_graphs`,
-reference GraphGenerator.py:99-161) for the §8(f) generation-round kernels.  Run in the build container:
+reference GraphGenerator.py:99-161) for the §8(f) generation-round kernels:
 
-    python tests/golden/make_generation_trace.py
+    GRAPHINVENT_REFERENCE=<GraphINVENT checkout> python tests/golden/make_generation_trace.py
 
 The unmodified reference `GraphGenerator` is imported with three stub modules (rdkit, MolecularGraph,
 parameters.constants -- SURVEY.md Appendix C); the model is the reference GGNN with the shipped checkpoint on CPU.
@@ -59,7 +59,7 @@ def main(batch=96, seed=7):
     import GraphGenerator as GG     # the unmodified reference module
     torch.manual_seed(seed)
     net = refimpl.build(O.make_constants("GGNN"))
-    net.load_state_dict(torch.load(os.path.join(HERE, "_local", "pretrained_model.pth"), map_location="cpu",
+    net.load_state_dict(torch.load(os.path.join(refimpl.DATA, "fine-tuning", "gdb13_1K-debug", "pretrained_model.pth"), map_location="cpu",
                                    weights_only=False))
     net.eval()
     draws, liks = [], []

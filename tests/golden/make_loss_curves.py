@@ -3,7 +3,7 @@ Golden training curves: the UNMODIFIED reference modules (CPU fp32) trained for 
 `Workflow.train_epoch` (Workflow.py:785-796: zero_grad -> forward -> KL loss -> backward -> Adam step, then the
 OneCycleLR step of Workflow.py:245-261) on the tiny-dims fixture batches of `small_<MODEL>.npz`.
 
-    python tests/golden/make_loss_curves.py        # build container only (needs /root/reference)
+    GRAPHINVENT_REFERENCE=<GraphINVENT checkout> python tests/golden/make_loss_curves.py
 
 Output `loss_curves.npz`: per model the 50 losses and the final logits.  SURVEY.md 8c lists "loss curve over 50 Adam
 steps within 1e-4" among the tolerances to hold.

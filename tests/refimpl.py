@@ -1,17 +1,19 @@
 """
-Loader for the UNMODIFIED reference modules (`/root/reference/graphinvent/gnn`), used
-only to pin the oracle: by `tests/golden/make_golden.py` (fixture generation) and by
-the live-reference tests, which skip when `/root/reference` is not mounted (it is
-absent on the GPU box).  Recipe = SURVEY.md Appendix C: `gnn/*` imports only torch.
+Loader for the UNMODIFIED reference modules (`graphinvent/gnn` of a GraphINVENT checkout), used only by the
+fixture generators under `tests/golden/` to pin the oracle.  The checkout is found through the environment variable
+GRAPHINVENT_REFERENCE (the repository root of MolecularAI/GraphINVENT); the test-suite itself never imports it.
+Recipe = SURVEY.md Appendix C: `gnn/*` imports only torch.
 """
 import os
 import sys
 
-REF_ROOT = "/root/reference/graphinvent"
+REPO = os.environ.get("GRAPHINVENT_REFERENCE", "")
+REF_ROOT = os.path.join(REPO, "graphinvent")
+DATA = os.path.join(REPO, "data")
 
 
 def available():
-    return os.path.isdir(os.path.join(REF_ROOT, "gnn"))
+    return bool(REPO) and os.path.isdir(os.path.join(REF_ROOT, "gnn"))
 
 
 def load():

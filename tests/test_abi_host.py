@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.conftest import MODELS, ROOT, load_small, pretrained_path
+from tests.conftest import MODELS, ROOT, load_small, pretrained_like_state_dict
 
 
 def test_header_symbols_are_exported_and_bound():
@@ -88,12 +88,10 @@ def test_modules_refuse_cpu_tensors_and_submodule_calls():
 
 
 def test_reference_checkpoint_loads_by_name():
-    path = pretrained_path()
-    if path is None:
-        pytest.skip("tests/golden/_local/pretrained_model.pth absent")
+    """the shipped checkpoint's tensor names, order and shapes (tests/golden/checkpoint_stats.npz)"""
     from graphinvent_b200.gnn import mpnn
     from oracle import mpnn_oracle as O
-    sd = torch.load(path, map_location="cpu", weights_only=False)
+    sd = pretrained_like_state_dict()
     net = mpnn.create(O.make_constants("GGNN"))
     missing, unexpected = net.load_state_dict(sd, strict=True)
     assert not missing and not unexpected
@@ -141,14 +139,14 @@ def test_synthetic_generator_matches_survey_statistics():
 
 
 def test_raw_hdf5_reader_matches_the_golden_rows():
+    """gdb13_1K/train.h5 of the reference, cut to its header and first 16 rows (tests/golden/make_golden.py)"""
     import os
     from graphinvent_b200 import data
-    path = "/root/reference/data/pre-training/gdb13_1K/train.h5"
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not mounted")
+    path = os.path.join(ROOT, "tests", "golden", "gdb13_train_excerpt.h5")
+    assert open(path, "rb").read(8) == b"\x89HDF\r\n\x1a\n"
     nodes, edges, apds = data.read_hdf5_raw(path, 13, 8, 3, 625)
     z = np.load(os.path.join(ROOT, "tests", "golden", "gdb13_rows.npz"))
-    assert nodes.shape == (12000, 13, 8) and edges.shape == (12000, 13, 13, 3) and apds.shape == (12000, 625)
-    assert (nodes[:256] == z["nodes"]).all() and (edges[:256] == z["edges"]).all() and (apds[:256] == z["apds"]).all()
+    assert nodes.shape == (16, 13, 8) and edges.shape == (16, 13, 13, 3) and apds.shape == (16, 625)
+    assert (nodes == z["nodes"][:16]).all() and (edges == z["edges"][:16]).all() and (apds == z["apds"][:16]).all()
     with pytest.raises(ValueError):
         data.read_hdf5_raw(path, 13, 8, 3, 624)

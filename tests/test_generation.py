@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.conftest import GOLDEN, pretrained_path
+from tests.conftest import GOLDEN
 
 
 def _trace():
@@ -132,31 +132,6 @@ def test_replay_reproduces_the_reference_generator_bit_exactly():
     assert torch.equal(gen.edges.cpu().to(torch.int8), torch.from_numpy(z["final_edges"]))
     assert torch.equal(gen.n_nodes.cpu().to(torch.int8), torch.from_numpy(z["final_n_nodes"]))
     assert torch.equal(gen.likelihoods.cpu(), torch.from_numpy(z["final_likelihoods"]))
-
-
-@pytest.mark.gpu
-def test_sampling_with_the_pretrained_checkpoint_builds_molecules():
-    path = pretrained_path()
-    if path is None:
-        pytest.skip("tests/golden/_local/pretrained_model.pth absent")
-    from graphinvent_b200.config import make_constants
-    from graphinvent_b200.generation import GraphGenerator
-    from graphinvent_b200.gnn import mpnn
-    C = make_constants("GGNN")
-    net = mpnn.create(C)
-    net.load_state_dict(torch.load(path, map_location="cpu", weights_only=False))
-    net = net.cuda().eval()
-    gen = GraphGenerator(net, batch_size=256, n_atom_types=5, n_formal_charge=3)
-    g = torch.Generator(device="cuda").manual_seed(0)
-    (nodes, edges, n_nodes), flat, final, proper = gen.sample(generator=g)
-    assert nodes.shape == (256, 13, 8) and edges.shape == (256, 13, 13, 3)
-    assert torch.isfinite(final).all() and (flat > 0).all()
-    # same statistics as the reference run that made the trace (mean 10.4 atoms, 69 % properly terminated)
-    assert 8.0 <= n_nodes.float().mean().item() <= 12.5
-    assert proper.float().mean().item() >= 0.45
-    atoms = (nodes.sum(-1) > 0).sum(-1)
-    assert torch.equal(atoms.to(torch.int8), n_nodes)
-    assert torch.equal(edges, edges.transpose(1, 2))
 
 
 @pytest.mark.gpu

@@ -2,7 +2,8 @@
 with autograd through the whole rollout (Workflow.learning_step, Workflow.py:569-612).
 
 Pin: tests/golden/generation_rl_trace.npz, recorded from the unmodified reference by
-tests/golden/make_generation_rl_trace.py (agent = shipped GGNN checkpoint, prior = checkpoint + seeded noise): draws
+tests/golden/make_generation_rl_trace.py (agent = conftest.pretrained_like_state_dict(), prior = those weights + seeded
+noise, draws of a rollout of the shipped trained checkpoint): draws
 and both likelihood streams of every round, final buffers, log-likelihoods, the loss of compute_loss_component and the
 gradient norms of both models."""
 import copy
@@ -13,7 +14,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.conftest import GOLDEN, pretrained_path
+from tests.conftest import GOLDEN, pretrained_like_state_dict
 from tests.test_generation import _action_stream
 
 N, A, CH, EF = 13, 5, 3, 3
@@ -21,6 +22,13 @@ N, A, CH, EF = 13, 5, 3, 3
 
 def _trace():
     return np.load(os.path.join(GOLDEN, "generation_rl_trace.npz"))
+
+
+def _trace_pretrained_like():
+    """the trace's draws and buffers with what the reference computed for conftest.pretrained_like_state_dict()"""
+    z = dict(_trace())
+    z.update(np.load(os.path.join(GOLDEN, "generation_rl_trace_pretrained_like.npz")))
+    return z
 
 
 def test_rl_oracle_replays_the_reference_rl_trace_bit_exactly():
@@ -161,21 +169,17 @@ class _OracleModel(torch.nn.Module):
 
 def test_rl_generator_with_oracle_models_reproduces_the_reference_trace(monkeypatch):
     """end to end on CPU: this package's GraphGeneratorRL (round kernel played by the generation oracle, models
-    played by the MPNN oracle with the shipped checkpoint) replays the reference's draws and must land on the
+    played by the MPNN oracle with the checkpoint-shaped weights) replays the reference's draws and must land on the
     reference's own numbers -- both likelihood streams, the log-likelihoods, the RL loss and the gradients that
     flow back through all 16 rounds into both models"""
-    from tests.conftest import pretrained_path
-    path = pretrained_path()
-    if path is None:
-        pytest.skip("tests/golden/_local/pretrained_model.pth absent")
     from oracle import mpnn_oracle as O
     from tests import hostshim
     from graphinvent_b200.config import make_constants
     from graphinvent_b200.generation import GraphGeneratorRL
     hostshim.install_generation_shims(monkeypatch)
-    z = _trace()
+    z = _trace_pretrained_like()
     B, n_gen, R = int(z["batch"]), int(z["n_generated"]), int(z["rounds"])
-    sd = torch.load(path, map_location="cpu", weights_only=False)
+    sd = pretrained_like_state_dict()
     g = torch.Generator().manual_seed(int(z["prior_seed"]))
     sd_prior = {k: v + float(z["prior_noise"]) * torch.randn(v.shape, generator=g) for k, v in sd.items()}
     C = O.make_constants("GGNN")
@@ -201,6 +205,6 @@ def test_rl_generator_with_oracle_models_reproduces_the_reference_trace(monkeypa
         for k, p in zip(net.names, net.params):
             assert abs(p.grad.norm().item() - ref[k]) <= 1e-3 * ref[k] + 1e-5 * total, (tag, k)
             key = f"grad_{tag}/{k}"
-            if key in z.files:
+            if key in z:
                 want = torch.from_numpy(z[key])
                 assert (p.grad - want).norm().item() <= 1e-3 * want.norm().item() + 1e-5 * total, (tag, k)

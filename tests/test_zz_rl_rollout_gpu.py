@@ -9,13 +9,20 @@ import numpy as np
 import pytest
 import torch
 
-from tests.conftest import GOLDEN, MODELS, load_small, pretrained_path
+from tests.conftest import GOLDEN, MODELS, load_small, pretrained_like_state_dict
 
 A, CH = 5, 3
 
 
 def _trace():
     return np.load(os.path.join(GOLDEN, "generation_rl_trace.npz"))
+
+
+def _trace_pretrained_like():
+    """the trace's draws and buffers with what the reference computed for conftest.pretrained_like_state_dict()"""
+    z = dict(_trace())
+    z.update(np.load(os.path.join(GOLDEN, "generation_rl_trace_pretrained_like.npz")))
+    return z
 
 
 def _perturbed(sd, seed, noise):
@@ -28,15 +35,12 @@ def test_rl_rollout_replay_matches_the_reference_trace():
     """the reference's draws replayed through the sm_100a path: identical molecules, the reference's two likelihood
     streams / log-likelihoods / loss, and the gradient the RL step back-propagates through all rounds of the rollout
     into BOTH models (one fused backward per round and model)"""
-    path = pretrained_path()
-    if path is None:
-        pytest.skip("tests/golden/_local/pretrained_model.pth absent")
     from graphinvent_b200.config import make_constants
     from graphinvent_b200.generation import GraphGeneratorRL
     from graphinvent_b200.gnn import mpnn
-    z = _trace()
+    z = _trace_pretrained_like()
     B, n_gen, R = int(z["batch"]), int(z["n_generated"]), int(z["rounds"])
-    sd = torch.load(path, map_location="cpu", weights_only=False)
+    sd = pretrained_like_state_dict()
     C = make_constants("GGNN")
     agent, prior = mpnn.create(C), mpnn.create(C)
     agent.load_state_dict(sd)
@@ -82,7 +86,7 @@ def test_rl_rollout_replay_matches_the_reference_trace():
             got_sq += gn * gn
             assert abs(gn - ref_norm[k]) <= 5e-2 * ref_norm[k] + 1e-3 * total, (tag, k, gn, ref_norm[k])
             key = f"grad_{tag}/{k}"
-            if key in z.files:
+            if key in z:
                 ref = torch.from_numpy(z[key])
                 assert (p.grad.cpu() - ref).norm().item() <= 5e-2 * ref.norm().item() + 1e-3 * total, (tag, k)
         assert abs(got_sq ** 0.5 - total) <= 2e-2 * total
